@@ -6,7 +6,8 @@ A step = one pass of the reference's timed region ("Batch-Time": after EncryptLa
 conv 5x5/2 (845 outputs) -> square -> dense 845->100 -> square -> dense 100->10, P plaintext moduli (default 2, the
 reference's configuration, `CryptoNets.cs:17`).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--plain-moduli 1|2]      B200 arm (one process per GPU under torchrun)
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--plain-moduli 1|2] [--dump-outputs DIR]
+                                                                                B200 arm (one process per GPU under torchrun)
   python bench.py --impl reference ...                                          CPU arm: the in-repo C++ oracle (the
         reference's C#/SEAL path cannot be built here) on all host cores, each step a bounded sample of the same workload.
 
@@ -288,6 +289,18 @@ def forward(layers, m):
     return m
 
 
+def dump_outputs(path, eng, scores):
+    """Writes what one step returned, so that two builds can be compared output for output on the same seeded inputs:
+    score_ciphertexts.npy, every residue word of the 10 score ciphertexts, shape (10, plaintext moduli, 2, coefficient moduli, N), and
+    scores.npy, their decryption, shape (images, 10).  Both float64, which holds residues below 2^53 exactly."""
+    words = np.stack([[v.vec.export_raw(ch, 0) for ch in range(eng.P)] for v in scores.vectors]).reshape(len(scores.vectors), eng.P, 2, eng.k, eng.N)
+    if int(words.max()) >= 1 << 53:
+        raise ValueError("ciphertext words need more than 53 bits: float64 would round them")
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "score_ciphertexts.npy"), words.astype(np.float64))
+    np.save(os.path.join(path, "scores.npy"), np.asarray(scores.Decrypt(), dtype=np.float64))
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -467,6 +480,8 @@ def run_b200(args):
                              "detail": cpu_info, "host": host_info()},
             "readme_anchor_images_per_s": 320.0,
         }
+        if args.dump_outputs:  # the last step of the timed loop above, its scores still held in `last`
+            dump_outputs(args.dump_outputs, eng, last)
     last.Dispose()
     xm.Dispose()
     f.Dispose()
@@ -567,12 +582,6 @@ def run_lola(args):
         ms = float(tms.item())
     images_per_step = 1 if shard else world
     value = args.steps * images_per_step / (ms * 1e-3)
-    if rank == 0:  # per-inference evaluator-operation counts: the CPU arm (`--impl reference --workload ...`) scales its per-op timings by them
-        try:
-            with open(os.path.join(ROOT, "profiles", "r02_opcounts_%s.json" % args.workload), "w") as fo:
-                json.dump(counts, fo)
-        except OSError:
-            pass
 
     # ---- e2e: the image's ciphertexts come from pinned host memory every step, the score ciphertexts go back to the host
     vecs = xm.vectors
@@ -679,8 +688,8 @@ def lola_cpu_estimate(workload, counts, threads=None):
 
 
 def run_reference_lola(args):
-    """CPU arm of a LoLa workload: needs the per-inference operation counts, which come from a recorded GPU run (profiles/) or, when none is
-    present, from the counts written next to this file by the B200 arm."""
+    """CPU arm of a LoLa workload: needs the per-inference operation counts, which come from a recorded GPU run (profiles/; the B200 arm
+    reports them as "operations_per_inference")."""
     path = os.path.join(ROOT, "profiles", "r02_opcounts_%s.json" % args.workload)
     counts = json.load(open(path))
     threads = host_threads()
@@ -773,7 +782,13 @@ def main():
                          "microbench = config 5 (one JSON line per case)")
     ap.add_argument("--microbench", action="store_true", help="same as --workload microbench")
     ap.add_argument("--shard-rows", action="store_true", help="lola_cifar on several GPUs: one image, the big dense layer's rows split over the ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="cryptonets on the B200: after the timed steps, write the score ciphertexts of the "
+                                                          "last timed step and their decryption to DIR/*.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "cryptonets" or args.microbench):
+        ap.error("--dump-outputs covers the cryptonets workload on the B200")
     if args.microbench or args.workload == "microbench":
         run_microbench(args)
     elif args.impl == "reference":

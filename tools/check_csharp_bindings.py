@@ -3,10 +3,11 @@
 1. every prototype of include/cnhe.h has exactly one [DllImport] with the same name, the same number of parameters and, per
    parameter, a C# type the C type may marshal as (pointers -> IntPtr / arrays / out scalars, size_t -> UIntPtr, ...);
 2. every member of the reference's IVector / IMatrix / IFactory / IComputationEnvironment interfaces is implemented by the B200
-   classes (member names are read from /root/reference when it is present -- the build container -- else from the list below, which
-   tests/test_abi_exports.py keeps equal to the reference's).
+   classes (the lists below, which must equal the member names recorded from the reference's interface files in
+   tests/golden/reference_interfaces.json).
 
 Run directly (exit code 1 on a mismatch) or through tests/test_abi_exports.py."""
+import json
 import os
 import re
 import sys
@@ -103,21 +104,17 @@ def check():
     for name in imports:
         if name not in protos:
             errors.append("[DllImport] %s is not declared in include/cnhe.h" % name)
-    ref = "/root/reference/HE Wrapper"
-    for cls, iface, fallback in (("B200BfvVector", "IVector.cs", IVECTOR), ("B200BfvMatrix", "IMatrix.cs", IMATRIX), ("B200BfvFactory", "IFactory.cs", IFACTORY),
-                                 ("B200BfvEnvironment", "IComputationEnvironment.cs", IENV)):
-        members = fallback
-        if os.path.exists(os.path.join(ref, iface)):
-            isrc = open(os.path.join(ref, iface), encoding="utf-8-sig").read()
-            start = isrc.index("interface " + iface[:-3])
-            block = isrc[start:isrc.index("\n    }", start)]
-            found = set(re.findall(r"\b([A-Z][A-Za-z]+)\s*(?:\(|\{\s*get)", block))
-            if set(fallback) - {"Dispose"} != found - {"Dispose"}:
-                errors.append("%s: member list in this script differs from the reference: %s" % (iface, sorted(found ^ (set(fallback) - {"Dispose"}))))
+    with open(os.path.join(ROOT, "tests", "golden", "reference_interfaces.json")) as f:
+        reference = json.load(f)
+    for cls, iface, members in (("B200BfvVector", "IVector", IVECTOR), ("B200BfvMatrix", "IMatrix", IMATRIX), ("B200BfvFactory", "IFactory", IFACTORY),
+                                ("B200BfvEnvironment", "IComputationEnvironment", IENV)):
+        found = set(reference[iface])
+        if set(members) != found:
+            errors.append("%s: member list in this script differs from the reference: %s" % (iface, sorted(found ^ set(members))))
         body = class_body(src, cls)
         for m in members:
             if not re.search(r"\bpublic\b[^;{=]*\b%s\b\s*(\(|\{|=>|;)" % m, body) and not re.search(r"\bpublic\b[^;{(]*\b%s\b" % m, body):
-                errors.append("%s does not implement %s.%s" % (cls, iface[:-3], m))
+                errors.append("%s does not implement %s.%s" % (cls, iface, m))
     return errors, len(protos)
 
 
